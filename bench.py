@@ -38,7 +38,7 @@ CONFIGS = {
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="timed steps (each of the two timed windows)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS))
@@ -49,7 +49,13 @@ def parse():
                          "views through the query encoder, in-batch negatives, no queue / momentum encoder)")
     ap.add_argument("--prefetch", type=int, default=4, choices=[1, 2, 3, 4, 5, 6, 8],
                     help="batches the sampler/eigensolver streams run ahead of the training stream")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (loss, embeddings, weights, queue, "
+                         "its batch) to DIR/<name>.npy, under 64 MB in all; same arguments, same inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def workload_name(cfg, n_gpus):
@@ -366,6 +372,8 @@ def run_ours(args, cfg):
     for b_ in eng.bufs:
         b_.check_flags()
     stats = eng.read_stats()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng)                  # before the e2e steps below change the state
     samp_ms = sum(a.elapsed_time(b) for a, b, _ in samp_ev) / len(samp_ev)
     eig_ms = sum(b.elapsed_time(c) for _, b, c in samp_ev) / len(samp_ev)
     n_sum, m_sum, t_sum, deg_sum = [float(x) / args.steps for x in cnt_acc.tolist()]
@@ -479,6 +487,46 @@ def run_ours(args, cfg):
         emit(line)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_ARRAY_BYTES = 4 << 20          # per array: 14 arrays at most, so a dump stays under 64 MB
+
+
+def dump_outputs(out_dir, eng):
+    """Write what the engine's last step computed as out_dir/<name>.npy, so that two builds can be compared
+    output for output (the inputs depend only on the command line): `loss`, `prob`, `grad_norm`; the query
+    and key embeddings `feat_q`, `feat_k`; the float entries of the encoder's state_dict after the update,
+    flattened in state_dict order (`model_state`; MoCo: also `ema_state` and the queue `memory`); the batch
+    the step trained on, per view v in q, k: `node_off_v` (ego-net offsets), `nodes_v` (parent-graph id of
+    every ego-net node) and `pos_v` (positional features).  Integer outputs are stored as float64, the rest
+    as float32.  An array larger than DUMP_ARRAY_BYTES keeps every s-th row, s the smallest stride that fits.
+    Two runs of one build give the same batch bit for bit, but the floats differ where kernels sum in a varying
+    order, so compare them with a tolerance: between two c2 runs on a B200 (1000 W) the largest difference was
+    1.7e-3, in a BatchNorm running variance; 4e-5 in the embeddings."""
+    import numpy as np
+    import torch
+
+    def flat_state(model):
+        return torch.cat([v.reshape(-1).float() for v in model.state_dict().values() if v.is_floating_point()])
+
+    buf, B = eng.cur_buf, eng.B
+    loss, prob, grad_norm = eng.stats[:3].tolist()
+    out = {"loss": np.float32(loss), "prob": np.float32(prob), "grad_norm": np.float32(grad_norm),
+           "feat_q": eng.feat_q, "feat_k": eng.feat_k, "model_state": flat_state(eng.model)}
+    if eng.moco:
+        out["ema_state"] = flat_state(eng.model_ema)
+        out["memory"] = eng.contrast.memory
+    for v, name in enumerate(("q", "k")):
+        n = int(buf.node_off[v, B])
+        out["node_off_" + name] = buf.node_off[v].double()
+        out["nodes_" + name] = buf.orig_id[v, :n].double()
+        out["pos_" + name] = buf.pos[v, :n]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        a = a.detach().cpu().numpy() if torch.is_tensor(a) else a
+        if a.nbytes > DUMP_ARRAY_BYTES:
+            a = a[::-(-a.nbytes // DUMP_ARRAY_BYTES)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def eigensolver_report(buf, eig_ms):

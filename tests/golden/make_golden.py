@@ -41,12 +41,24 @@ import gcc.models.graph_encoder as ref_ge  # noqa: E402
 import gcc.utils.misc as ref_misc  # noqa: E402
 
 KEY = 0x5EED5EED
+PART_BYTES = 900_000        # no fixture file may exceed 1 MB
 
 
 def save(name, **arrays):
-    path = os.path.join(HERE, name)
-    np.savez_compressed(path, **arrays)
-    print("wrote", path, "(%d arrays)" % len(arrays))
+    """tests/golden/<name>.npz; a fixture holding more than PART_BYTES of arrays is written as parts
+    <name>.0.npz, <name>.1.npz, ... in key order (the `golden` fixture of tests/conftest.py merges them)."""
+    parts, size = [{}], 0
+    for k, v in arrays.items():
+        if parts[-1] and size + v.nbytes > PART_BYTES:
+            parts.append({})
+            size = 0
+        parts[-1][k] = v
+        size += v.nbytes
+    stem = os.path.join(HERE, name[:-len(".npz")])
+    paths = [stem + ".npz"] if len(parts) == 1 else ["%s.%d.npz" % (stem, i) for i in range(len(parts))]
+    for path, part in zip(paths, parts):
+        np.savez_compressed(path, **part)
+        print("wrote", path, "(%d arrays)" % len(part))
 
 
 # ----------------------------------------------------------------------------- #

@@ -1,7 +1,6 @@
 """GPU: the finetune path (SURVEY.md section 8 row N4) -- train.py:train_finetune / test_finetune through the
-device kernels against tests/golden/train_finetune_golden.npz (produced by the REAL reference train_finetune),
+device kernels against tests/golden/train_finetune_golden.*.npz (produced by the REAL reference train_finetune),
 and the labeled datasets (ego-net and whole-graph batches) against the CPU oracle."""
-import os
 import types
 
 import numpy as np
@@ -9,8 +8,6 @@ import pytest
 import torch
 
 pytestmark = pytest.mark.gpu
-
-G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def _encoder(H, L):
@@ -44,13 +41,13 @@ def _fixture_batch(z, prefix):
     return buf
 
 
-def test_finetune_vs_reference_golden():
+def test_finetune_vs_reference_golden(golden):
     import train
     from gcc_b200.datasets.data_util import BatchedSubgraphs
-    z = np.load(os.path.join(G, "train_finetune_golden.npz"))
+    z = golden("train_finetune_golden")
     L, H, S, C = int(z["num_layer"]), int(z["hidden"]), int(z["num_steps"]), int(z["num_classes"])
     model = _encoder(H, L)
-    model.load_state_dict({k[5:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("init/")})
+    model.load_state_dict({k[5:]: torch.from_numpy(z[k]) for k in z if k.startswith("init/")})
     model = model.cuda()
     model.dropout_key = int(z["key"])
     out_layer = torch.nn.Linear(H, C)
@@ -71,7 +68,7 @@ def test_finetune_vs_reference_golden():
         assert np.isclose(loss, z["losses"][st], rtol=1e-3), (st, loss, z["losses"][st])
         assert np.isclose(f1, z["f1"][st]), (st, f1, z["f1"][st])
         sd = {k: v.cpu().numpy() for k, v in model.state_dict().items()}
-        for k in z.files:
+        for k in z:
             if k.startswith("s%d_model/" % st):
                 name = k.split("/", 1)[1]
                 if ("mlp.linears" in name and name.endswith("bias")) or \

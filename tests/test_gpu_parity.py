@@ -221,16 +221,16 @@ def _golden_batch(z, st):
 
 
 @pytest.mark.parametrize("tag", ["moco", "e2e"])
-def test_train_step_vs_reference_golden(tag):
+def test_train_step_vs_reference_golden(tag, golden):
     """The module-level API (GraphEncoder + MemoryMoCo + NCESoftmaxLoss + torch Adam, wired exactly
-    like the reference's train_moco) reproduces tests/golden/train_*_golden.npz, which was produced
+    like the reference's train_moco) reproduces tests/golden/train_*_golden.*.npz, which was produced
     by the REAL reference train_moco: losses, weights after Adam, EMA weights, queue."""
     from gcc_b200.contrastive.criterions import NCESoftmaxLoss, NCESoftmaxLossNS
     from gcc_b200.contrastive.memory_moco import MemoryMoCo
     from gcc_b200.datasets.data_util import BatchedSubgraphs
     from gcc_b200.models import GraphEncoder
     from gcc_b200.utils.misc import warmup_linear
-    z = np.load(os.path.join(G, "train_%s_golden.npz" % tag))
+    z = golden("train_%s_golden" % tag)
     L, H, S, K, moco = int(z["num_layer"]), int(z["hidden"]), int(z["num_steps"]), int(z["K"]), bool(z["moco"])
 
     def mk():
@@ -240,7 +240,7 @@ def test_train_step_vs_reference_golden(tag):
                             norm=True, gnn_model="gin", degree_input=True)
 
     model, model_ema = mk(), mk()
-    init = {k[5:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("init/")}
+    init = {k[5:]: torch.from_numpy(z[k]) for k in z if k.startswith("init/")}
     model.load_state_dict(init)
     model_ema.load_state_dict(init)
     model, model_ema = model.cuda(), model_ema.cuda()
@@ -278,7 +278,7 @@ def test_train_step_vs_reference_golden(tag):
                 p2.data.mul_(0.999).add_(p1.detach().data, alpha=1 - 0.999)
         assert np.isclose(loss.item(), z["losses"][st], rtol=1e-3), (st, loss.item(), z["losses"][st])
         sd = {k: v.cpu().numpy() for k, v in model.state_dict().items()}
-        for k in z.files:
+        for k in z:
             if k.startswith("s%d_model/" % st):
                 name = k.split("/", 1)[1]
                 if ("mlp.linears" in name and name.endswith("bias")) or \
@@ -290,7 +290,7 @@ def test_train_step_vs_reference_golden(tag):
     if moco:
         assert contrast.index == int(z["final_index"])
         sde = {k: v.cpu().numpy() for k, v in model_ema.state_dict().items()}
-        for k in z.files:
+        for k in z:
             if k.startswith("s%d_ema/" % (S - 1)):
                 name = k.split("/", 1)[1]
                 if name.endswith("running_mean") and "apply_func" in name:

@@ -64,7 +64,7 @@ def test_generation_budget_uses_the_plain_degree():
             assert budget_for_degree(deg, hops, rp) == max(hops, int(((deg ** 0.75) * math.e / (math.e - 1) / rp) + 0.5))
 
 
-def test_param_layout_matches_c_layout_and_reference_state_dict():
+def test_param_layout_matches_c_layout_and_reference_state_dict(golden):
     from gcc_b200 import _capi
     from gcc_b200.models import GraphEncoder
     from gcc_b200.models import layout as glayout
@@ -82,13 +82,13 @@ def test_param_layout_matches_c_layout_and_reference_state_dict():
         assert lay.wp[L - 1] == sl["gnn.linears_prediction.%d.weight" % (L - 1)][0]
         assert lay.emb == sl["degree_embedding.weight"][0]
     # same torch seed as the golden run -> identical initial weights, identical state_dict keys/order
-    z = np.load(os.path.join(G, "train_moco_golden.npz"))
+    z = golden("train_moco_golden")
     torch.manual_seed(11)
     m = GraphEncoder(positional_embedding_size=32, max_node_freq=16, max_edge_freq=16, max_degree=512,
                      freq_embedding_size=16, degree_embedding_size=16, output_dim=64, node_hidden_dim=64,
                      edge_hidden_dim=64, num_layers=5, num_step_set2set=6, num_layer_set2set=3, norm=True,
                      gnn_model="gin", degree_input=True)
-    ref_keys = [k[5:] for k in z.files if k.startswith("init/")]
+    ref_keys = [k[5:] for k in z if k.startswith("init/")]
     sd = m.state_dict()
     assert list(sd.keys()) == ref_keys
     for k in ref_keys:
