@@ -75,6 +75,14 @@ _PROTOS = {
     "gccb_tc_gemm_bf16": (C.c_int, [p, p, C.c_int32, C.c_int32, C.c_int32, p, p, C.c_float, p, p, C.c_int32, p,
                                     C.c_int32, p, p]),
     "gccb_cast_bf16": (C.c_int, [p, C.c_int32, C.c_int32, C.c_int32, p, C.c_int32, C.c_int32, C.c_int32, p, p]),
+    "gccb_logreg_ovr_workspace": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32, C.c_int32]),
+    "gccb_logreg_ovr": (C.c_int, [p, p, p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_int32,
+                                  C.c_double, p, p, p, p, p, C.c_size_t, p]),
+    "gccb_svc_ovo_workspace": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32]),
+    "gccb_svc_ovo": (C.c_int, [p, p, p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_double,
+                               C.c_int64, p, p, p, p, p, p, p, p, C.c_size_t, p]),
+    "gccb_sim_rank_workspace": (C.c_size_t, [C.c_int32, C.c_int32]),
+    "gccb_sim_rank": (C.c_int, [p, p, C.c_int32, p, p, C.c_int32, p, p, C.c_size_t, p]),
 }
 
 SYMBOLS = tuple(_PROTOS)

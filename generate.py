@@ -7,8 +7,13 @@ same `model` state_dict keys), walks two ego-nets from EVERY node of the target 
 (BatchNorm running statistics, no dropout) and saves (f(q) + f(k)) / 2 as `<model_folder>/<name>.npy`
 (generate.py:48-53,133-134).  The reference batches the whole dataset into ONE batch (:90); here
 the nodes go through in `--batch-size` chunks -- eval-mode encoding is per-graph, so the result is
-the same.  `--dataset` is an .npz CSR (indptr, indices) or `synthetic-<kind>`: the reference's named
-datasets need the network / DGL (SURVEY.md 8f N2, N3).
+the same.  `--dataset` is an .npz CSR (indptr, indices), `synthetic-<kind>`, or one of the reference's
+names whose files are under ./data: the airport / h-index edge lists, the PanTher graphs (kdd, icdm, sigir,
+cikm, sigmod, icde; multi-edges collapsed) and the five TU graph-classification sets.
+
+Graph-classification inputs (a TU name, or an .npz with graph_sizes) export ONE embedding per graph
+(generate.py:74-81): the eval-mode encoding of the whole graph, seeded at its max-degree node.  Both of
+the reference's views are the whole graph, so their mean is that encoding.
 """
 import argparse
 import os
@@ -16,7 +21,7 @@ import os
 import numpy as np
 import torch
 
-from gcc_b200.datasets import synthetic
+from gcc_b200.datasets import labeled, panther, synthetic
 from gcc_b200.datasets.graph_dataset import NodeClassificationDataset
 from gcc_b200.models import GraphEncoder
 
@@ -44,10 +49,41 @@ def test_moco(train_loader, model, opt):
     return torch.cat(chunks)
 
 
+def is_graph_dataset(name):
+    """A TU name or an .npz of a disjoint union with graph_sizes."""
+    if name.endswith(".npz"):
+        with np.load(name) as z:
+            return "graph_sizes" in z
+    return name in labeled.GRAPH_CLASSIFICATION_DSETS
+
+
+def graph_embeddings(name, encoder, batch_size, positional_embedding_size=32):
+    """One eval-mode embedding per whole graph, in dataset order."""
+    ds = labeled.GraphClassificationDatasetLabeled(name, positional_embedding_size=positional_embedding_size,
+                                                   device=encoder_device(encoder), batch_size=batch_size)
+    encoder.eval()
+    chunks = []
+    with torch.no_grad():
+        for graph_q, _ in ds.batches():
+            chunks.append(encoder(graph_q).cpu())
+    return torch.cat(chunks)
+
+
+def encoder_device(encoder):
+    return next(encoder.parameters()).device
+
+
 def resolve_graph(name, nodes, edges):
-    """`--dataset`: an .npz path is passed through; synthetic-chunglu / synthetic-er are generated."""
+    """`--dataset`: an .npz path is passed through; the reference's node datasets are read from ./data;
+    synthetic-chunglu / synthetic-er are generated."""
     if name.endswith(".npz"):
         return name
+    if name in labeled._EDGELIST_NAMES:
+        e = labeled.Edgelist(*labeled._EDGELIST_NAMES[name])
+        return labeled.graph_from_edge_index(e.data.edge_index.numpy())
+    if name in panther.PANTHER_NAMES:
+        e = panther.SSSingleDataset(panther.PANTHER_ROOT, name)
+        return labeled.graph_from_edge_index(e.data.edge_index.numpy())
     if name.endswith("chunglu"):
         return synthetic.chung_lu(nodes, edges, 0.5, seed=0)
     return synthetic.erdos_renyi(nodes, edges, seed=0)
@@ -72,12 +108,15 @@ def main(args_test):
     encoder = encoder.to(opt.device)
     del ckpt
 
-    nodes = NodeClassificationDataset(
-        dataset=resolve_graph(args_test.dataset, args_test.graph_nodes, args_test.graph_edges),
-        rw_hops=opt.rw_hops, subgraph_size=opt.subgraph_size, restart_prob=opt.restart_prob,
-        positional_embedding_size=opt.positional_embedding_size, device=opt.device,
-        seed=getattr(opt, "seed", 0), batch_size=args_test.batch_size)
-    emb = test_moco(nodes, encoder, opt)
+    if is_graph_dataset(args_test.dataset):
+        emb = graph_embeddings(args_test.dataset, encoder, args_test.batch_size, opt.positional_embedding_size)
+    else:
+        nodes = NodeClassificationDataset(
+            dataset=resolve_graph(args_test.dataset, args_test.graph_nodes, args_test.graph_edges),
+            rw_hops=opt.rw_hops, subgraph_size=opt.subgraph_size, restart_prob=opt.restart_prob,
+            positional_embedding_size=opt.positional_embedding_size, device=opt.device,
+            seed=getattr(opt, "seed", 0), batch_size=args_test.batch_size)
+        emb = test_moco(nodes, encoder, opt)
 
     stem = os.path.basename(args_test.dataset)
     stem = stem[:-4] if stem.endswith(".npz") else stem
@@ -91,7 +130,9 @@ if __name__ == "__main__":
     ap = argparse.ArgumentParser("inference export: node embeddings from a pretraining checkpoint")
     ap.add_argument("--load-path", type=str, required=True, help="path to load model")
     ap.add_argument("--dataset", type=str, default="synthetic-er",
-                    help=".npz CSR file (indptr, indices) or synthetic-er / synthetic-chunglu")
+                    help=".npz CSR file (indptr, indices; graph_sizes + graph_labels for one embedding per graph), "
+                         "synthetic-er / synthetic-chunglu, or a dataset name of the reference with its files "
+                         "under ./data")
     ap.add_argument("--graph-nodes", type=int, default=2000, help="size of a synthetic target graph")
     ap.add_argument("--graph-edges", type=int, default=10000)
     ap.add_argument("--batch-size", type=int, default=256, help="nodes encoded per launch group")

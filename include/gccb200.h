@@ -255,6 +255,48 @@ int gccb_tc_gemm_bf16(const void* A, const void* B, int32_t M_cap, int32_t N, in
 int gccb_cast_bf16(const float* src, int32_t rows, int32_t cols, int32_t lds, void* dst, int32_t rows_pad,
                    int32_t cols_pad, int32_t transpose, const int32_t* rows_dev, gccb_stream_t stream);
 
+/* ---- frozen-embedding evaluation (csrc/downstream.cu) -----------------------------------------------
+ * k-fold scoring of exported embeddings; every (fold, class) or (fold, class pair) problem of a call is
+ * solved in ONE launch, one CTA each.  X: float32 [n][d] (the .npy generate.py writes); label: int32 [n]
+ * in 0..n_classes-1; fold: int32 [n] in 0..n_folds-1 (row i is a test row of fold fold[i] and a training
+ * row of every other fold).  Arithmetic that decides a prediction is fp64.
+ * status (per problem): 0 converged, 1 iteration cap reached, 2 (logreg) no further decrease at fp64
+ * resolution, 3 / 4 (logreg) class absent from / the only class of the training fold: constant
+ * probability 0 / 1 (sklearn's _ConstantPredictor).                                                    */
+
+/* One-vs-rest L2 logistic regression (gcc/tasks/node_classification.py:54-90, TopKRanker(
+ * LogisticRegression(C))): problem p = fold*n_classes + class minimises 1/2|w|^2 + C sum log(1 + exp(-s(w.x+b)))
+ * over its training rows (intercept unpenalised) by Newton's method with backtracking; stops when
+ * lambda^2/2 <= tol * max(1, objective) (Newton decrement) or after max_iter steps.
+ * weights: double [n_folds*n_classes][d+1] (w, then b).  prob (optional): double [n][n_classes], the
+ * sigmoid probability of every class under the row's own fold model.  pred: int32 [n], the top-1 class
+ * (a tie, e.g. probabilities saturated to 1.0, goes to the highest class index).                       */
+size_t gccb_logreg_ovr_workspace(int32_t n, int32_t d, int32_t n_classes, int32_t n_folds);
+int gccb_logreg_ovr(const float* X, const int32_t* label, const int32_t* fold, int32_t n, int32_t d,
+                    int32_t n_classes, int32_t n_folds, double C, int32_t max_iter, double tol,
+                    double* weights, double* prob, int32_t* pred, int32_t* status, void* workspace,
+                    size_t workspace_bytes, gccb_stream_t stream);
+
+/* RBF C-SVC, one-vs-one (gcc/tasks/graph_classification.py:46-66, SVC(C)): gamma = 1/(d var(X_train))
+ * per fold (gamma='scale'), libsvm's SMO with second-order working-set selection, stop when
+ * m(alpha) - M(alpha) < eps.  Pairs (ci < cj) in libsvm order, ci is the +1 class; problem
+ * p = fold*n_pairs + pair.  gamma: double [n_folds]; coef: double [P][n], y*alpha at the dataset row
+ * (0 elsewhere); rho, obj (dual objective): double [P]; dec (optional): double [n][n_pairs], decision
+ * values of every row under its own fold; pred: int32 [n], libsvm's vote (f > 0 votes for ci; a tie goes
+ * to the lowest class).  n_classes <= 64.  The workspace holds the n x n squared distances (fp32).   */
+size_t gccb_svc_ovo_workspace(int32_t n, int32_t n_classes, int32_t n_folds);
+int gccb_svc_ovo(const float* X, const int32_t* label, const int32_t* fold, int32_t n, int32_t d,
+                 int32_t n_classes, int32_t n_folds, double C, double eps, int64_t max_iter, double* gamma,
+                 double* coef, double* rho, double* obj, double* dec, int32_t* pred, int32_t* status,
+                 void* workspace, size_t workspace_bytes, gccb_stream_t stream);
+
+/* Similarity-search rank (gcc/tasks/similarity_search.py:40-70): rows E1[idx1[q]] and E2[idx2[q]]
+ * (q < m shared keys) are L2-normalised in fp64; rank[q] = number of c < m with
+ * score(q, c) > score(q, q), score = e1[q].e2[c].  Recall@k = mean(rank < k).                       */
+size_t gccb_sim_rank_workspace(int32_t m, int32_t d);
+int gccb_sim_rank(const float* E1, const float* E2, int32_t d, const int32_t* idx1, const int32_t* idx2,
+                  int32_t m, int32_t* rank, void* workspace, size_t workspace_bytes, gccb_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
